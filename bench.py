@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- LM iterations/sec on the batched SE3 pose graph of BASELINE.json, on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     (N>1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
 
 HEADLINE (value / e2e / roofline / cpu_baseline / parity): BASELINE.json's scaling configuration C5 -- sphere-like SE3 pose graph,
@@ -47,6 +47,8 @@ C2_POSES, C2_BATCH = 256, 256
 C2_WORKLOAD = ("C2: synthetic SE3 pose-graph (pose_graph_cube shape: 256 poses, loop_closure_ratio 0.2), batch=256 per GPU (weak), "
                "LM(10 it, adaptive+ellipsoidal damping) + CholeskyDenseSolver")
 CPU_SAMPLE_ITEMS = 32
+# --dump-outputs: the solution of a fixed, seeded sample of batch items (128 x 2 500 poses x 12 doubles = 31 MB; all 4096 would be 983 MB)
+DUMP_ITEMS, DUMP_SEED = 128, 0
 # sparse CPU arms: one process per batch item, as many items as the host has cores (bounded: 16..128) -- the reference's per-item loop on ALL cores
 C5_CPU_ITEMS = int(os.environ.get("THB_BENCH_CPU_ITEMS", str(max(16, min(os.cpu_count() or 16, 128)))))
 
@@ -139,6 +141,24 @@ def cpu_run(data, items, solver, iters=LM_ITERS):
     return dt, out, cores, (min(cores, items) if solver == "sparse" else used)
 
 
+def dump_outputs(path, values, info, names):
+    """--dump-outputs: what one LM solve of the timed path hands its caller, as float64 .npy files under `path`: per batch item the final
+    error, the iteration counts, and the status code (NonlinearOptimizerStatus value: 1 converged, 2 max iterations, -1 failed); and the
+    optimised poses ([items, poses, 3, 4]) of DUMP_ITEMS items drawn with DUMP_SEED (their indices in poses_sample_items.npy).  The inputs
+    are seeded, so two builds run with the same arguments can be compared file by file."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    B = info.last_err.shape[0]
+    items = np.sort(np.random.default_rng(DUMP_SEED).choice(B, size=min(B, DUMP_ITEMS), replace=False))
+    idx = torch.from_numpy(items).to(info.last_err.device)
+    poses = torch.stack([values[n].index_select(0, idx) for n in names], 1)
+    status = torch.tensor([s.value for s in info.status])
+    arrays = dict(last_err=info.last_err, converged_iter=info.converged_iter, best_iter=info.best_iter, status=status, poses_sample=poses,
+                  poses_sample_items=torch.from_numpy(items))
+    for name, t in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), t.detach().to(torch.float64).cpu().numpy())
+
+
 def make_c5_data(batch, seed, device="cpu"):
     from theseus_b200.datasets import pose_graph_sphere
     return pose_graph_sphere(C5_RINGS, C5_PER_RING, batch, seed=seed, device=device)
@@ -146,9 +166,9 @@ def make_c5_data(batch, seed, device="cpu"):
 
 # ------------------------------------------------------------------------------------------------ --impl reference
 def run_reference(args):
-    """--impl reference: the reference's own CPU algorithm for the headline workload (oracle port; /root/reference is Python and does
-    not travel to the GPU box), all host cores, rank 0 only.  Each step = the LM solve of a bounded sample (C5_CPU_ITEMS of the 4096
-    items); value = LM iterations/s of the 4096-batch assuming the reference's per-item loop scales linearly in the batch."""
+    """--impl reference: the reference's own CPU algorithm for the headline workload (numpy port in oracle/), all host cores, rank 0
+    only.  Each of the --steps timed steps = the LM solve of a bounded sample (C5_CPU_ITEMS of the 4096 items); value = LM iterations/s
+    of the 4096-batch assuming the reference's per-item loop scales linearly in the batch."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -161,8 +181,6 @@ def run_reference(args):
     for _ in range(args.steps):
         dt, _, cores, used = cpu_run(data, sample, "sparse")
         times.append(dt)
-        if sum(times) > 120.0:   # the whole run must end within a few minutes (one step = ~47 s on 128 cores)
-            break
     t_sample = float(np.mean(times))
     t_full = t_sample * C5_GLOBAL_BATCH / sample
     value = LM_ITERS / t_full
@@ -182,12 +200,22 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps of every timed leg (default: 10; 3 with --impl reference, whose step is one CPU solve of "
+                         "C5_CPU_ITEMS items, ~47 s on 128 cores)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-c2", action="store_true", help="skip the dense C2 leg reported beside the headline")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy (with --gpus N > 1: "
+                                                          "rank 0's shard only, so dumps are comparable between runs at the same N)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 3 if args.impl == "reference" else 10
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -265,6 +293,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     value = LM_ITERS * 1e3 / ms_step
     final_err = out["info"].last_err.clone()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out["values"], out["info"], names_pose)
 
     # ---- e2e: pinned host inputs -> device, public API, solution + error back to pinned host memory, every step ----
     host_poses, host_meas = data["poses"].pin_memory(), data["meas"].pin_memory()
@@ -285,7 +315,7 @@ def main():
         host_err.copy_(info.last_err, non_blocking=True)
         torch.cuda.current_stream().synchronize()
 
-    e2e_steps = max(2, min(args.steps, 5))
+    e2e_steps = args.steps
     step_e2e()
     ms_e2e = timed(step_e2e, e2e_steps) / e2e_steps
     h2d = (host_poses.numel() + host_meas.numel()) * 8 * world       # whole job, per step
@@ -378,7 +408,7 @@ def main():
     c2 = None
     if not args.no_c2:
         try:
-            c2 = dense_c2_leg(th, lib, _lib, device, rank, world, pg, timed, peak_tf, steps=min(args.steps, 5), with_cpu=(rank == 0 and world == 1 and not args.no_cpu_baseline))
+            c2 = dense_c2_leg(th, lib, _lib, device, rank, world, pg, timed, peak_tf, steps=args.steps, with_cpu=(rank == 0 and world == 1 and not args.no_cpu_baseline))
         except Exception as e:   # the leg is reported beside the headline: a failure there must not take the headline down
             c2 = dict(error=repr(e)[:300])
 
