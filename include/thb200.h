@@ -52,13 +52,26 @@ enum thb_cost_kind {
   THB_COST_LOCAL_VECTOR = 4, /* Difference on Vector/Point: e = x - target, J = I (geometry/vector.py) */
   THB_COST_BETWEEN_SE2 = 6,  /* Between with SE2 [B,4] = [x,y,cos,sin] (theseus/geometry/se2.py) */
   THB_COST_LOCAL_SE2 = 7,    /* Difference / Local with SE2 */
-  THB_COST_REPROJECTION = 5  /* theseus/embodied/measurements/reprojection.py:54-94: x0 = camera SE3, x1 = Point3,
+  THB_COST_REPROJECTION = 5, /* theseus/embodied/measurements/reprojection.py:54-94: x0 = camera SE3, x1 = Point3,
                                 aux = focal_length [Bf,1], aux2 = image_feature_point [Bi,2], aux3 = calib_k1, aux4 = calib_k2 */
+  /* theseus/embodied/collision/collision.py: e = max(eps - sdf(xy), 0), dim 1, x0 = pose (Point2 [B,2] / SE2 [B,4]);
+   * aux = sdf_origin [Bo,2], aux2 = sdf_data [Bs,sdf_rows,sdf_cols], aux3 = sdf_cell_size [Bc,1], aux4 = cost_eps [Be,1] */
+  THB_COST_COLLISION2D_POINT2 = 8,
+  THB_COST_COLLISION2D_SE2 = 9,
+  /* theseus/embodied/motionmodel/double_integrator.py:16-95: e = [pose1.local(pose2) - dt vel1 ; vel2 - vel1], dim 2 dof;
+   * x0 = pose1, x1 = vel1, x2 = pose2, x3 = vel2; aux = dt [Bd,1]; with THB_WEIGHT_GP aux2 = the weight's own dt [Bw,1].
+   * VECTOR: poses of Vector kind with dof 2 or 3 (Point2, Point3, Vector); SE2: poses SE2, velocities Vector dof 3. */
+  THB_COST_DOUBLE_INTEGRATOR_VECTOR = 10,
+  THB_COST_DOUBLE_INTEGRATOR_SE2 = 11
 };
 enum thb_robust_kind { THB_ROBUST_NONE = 0, THB_ROBUST_WELSCH = 1, THB_ROBUST_HUBER = 2 };
 enum thb_weight_kind {
   THB_WEIGHT_SCALE = 0,   /* theseus/core/cost_weight.py:60-93  (ScaleCostWeight, tensor [Bw,1]) */
-  THB_WEIGHT_DIAGONAL = 1 /* theseus/core/cost_weight.py:98-139 (DiagonalCostWeight, tensor [Bw,dim]) */
+  THB_WEIGHT_DIAGONAL = 1, /* theseus/core/cost_weight.py:98-139 (DiagonalCostWeight, tensor [Bw,dim]) */
+  /* theseus/embodied/motionmodel/double_integrator.py:98-175 (GPCostWeight): w = Qc_inv [Bq,d,d], the weight's dt in aux2 [Bw,1].
+   * Weighting is U e, U J with U = chol(W^T)^T, W = [[12/dt^3, -6/dt^2], [-6/dt^2, 4/dt]] (x) Qc_inv, formed in registers as
+   * (chol(M) (x) chol(Qc_inv^T))^T (the Cholesky factor is unique).  Accepted by the DOUBLE_INTEGRATOR kinds only (d <= 3). */
+  THB_WEIGHT_GP = 2
 };
 enum thb_var_kind { THB_VAR_SE3 = 0, THB_VAR_SO3 = 1, THB_VAR_VECTOR = 2, THB_VAR_SE2 = 3, THB_VAR_SO2 = 4 };
 
@@ -78,7 +91,8 @@ typedef struct thb_cost_group {
   /* Placement in the reference's batched-CSR Jacobian (theseus/optimizer/sparse_linearization.py:34-84): */
   const int64_t* a_off;    /* device [K]   offset of the cost function's first row in A_val (cost_function_row_block_starts) */
   const int32_t* a_stride; /* device [K]   entries per row (cost_function_stride) */
-  const int32_t* bp;       /* device [K,2] column offset of each variable's block inside a row (cost_function_block_pointers) */
+  const int32_t* bp;       /* device [K,nv] column offset of each variable's block inside a row (cost_function_block_pointers);
+                            * nv = 4 for the DOUBLE_INTEGRATOR kinds, 2 for every other kind (unused slots 0) */
   const int32_t* row0;     /* device [K]   first row of the cost function in b */
   /* further auxiliary tensors of schemas that need them (NULL otherwise) + their batch strides, device int32 [K,3] */
   const void* const* aux2;
@@ -91,6 +105,14 @@ typedef struct thb_cost_group {
   int32_t reserved0;
   const void* const* log_radius;
   const int32_t* bstride_lr;
+  /* Fields appended after the ones above (whose offsets are unchanged):
+   * third and fourth optimisation variable (DOUBLE_INTEGRATOR kinds: pose2, vel2) or NULL, their batch strides device int32 [K,2] */
+  const void* const* x2;
+  const void* const* x3;
+  const int32_t* bstride3;
+  /* grid shape [sdf_rows, sdf_cols] shared by every cost function of a COLLISION2D group (0 for other kinds) */
+  int32_t sdf_rows;
+  int32_t sdf_cols;
 } thb_cost_group;
 
 /* Fused residual + analytic Jacobian + weighting for every (cost function, batch item) of a group;

@@ -19,7 +19,8 @@ class CostGroup(C.Structure):
                 ("x0", c_vp), ("x1", c_vp), ("aux", c_vp), ("w", c_vp), ("bstride", c_vp),
                 ("a_off", c_vp), ("a_stride", c_vp), ("bp", c_vp), ("row0", c_vp),
                 ("aux2", c_vp), ("aux3", c_vp), ("aux4", c_vp), ("bstride2", c_vp),
-                ("robust_kind", c_i32), ("reserved0", c_i32), ("log_radius", c_vp), ("bstride_lr", c_vp)]
+                ("robust_kind", c_i32), ("reserved0", c_i32), ("log_radius", c_vp), ("bstride_lr", c_vp),
+                ("x2", c_vp), ("x3", c_vp), ("bstride3", c_vp), ("sdf_rows", c_i32), ("sdf_cols", c_i32)]
 
 
 class VarTable(C.Structure):

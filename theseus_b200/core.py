@@ -23,7 +23,10 @@ from .geometry import LieGroup, Manifold, Point2, Point3, SE2, SE3, SO2, SO3, Va
 # enum thb_cost_kind / thb_weight_kind (include/thb200.h)
 COST_BETWEEN_SE3, COST_LOCAL_SE3, COST_BETWEEN_SO3, COST_LOCAL_SO3, COST_LOCAL_VECTOR, COST_REPROJECTION = 0, 1, 2, 3, 4, 5
 COST_BETWEEN_SE2, COST_LOCAL_SE2 = 6, 7
-WEIGHT_SCALE, WEIGHT_DIAGONAL = 0, 1
+COST_COLLISION2D_POINT2, COST_COLLISION2D_SE2, COST_DOUBLE_INTEGRATOR_VECTOR, COST_DOUBLE_INTEGRATOR_SE2 = 8, 9, 10, 11
+WEIGHT_SCALE, WEIGHT_DIAGONAL, WEIGHT_GP = 0, 1, 2
+# kinds whose kernels have no fused robust loss: a RobustCostFunction around them takes the generic route
+_NO_FUSED_ROBUST = (COST_LOCAL_VECTOR, COST_COLLISION2D_POINT2, COST_COLLISION2D_SE2, COST_DOUBLE_INTEGRATOR_VECTOR, COST_DOUBLE_INTEGRATOR_SE2)
 
 
 def _shallow_clone_with_copied_vars(obj, attr_names, new_name):
@@ -332,7 +335,7 @@ class CostFunction:
         return self.aux_vars
 
     def _weight(self, err: torch.Tensor, jacs):
-        if self.weight.WEIGHT_KIND < 0:   # user-defined CostWeight
+        if self.weight.WEIGHT_KIND not in (WEIGHT_SCALE, WEIGHT_DIAGONAL):   # user-defined or full-matrix (GPCostWeight) CostWeight
             if jacs is None:
                 return None, self.weight.weight_error(err)
             wj, we = self.weight.weight_jacobians_and_error(list(jacs), err)
@@ -630,7 +633,7 @@ class RobustCostFunction(CostFunction):
     def schema(self):
         kind, aux = self.cost_function.schema()
         aux = list(aux) if isinstance(aux, (list, tuple)) else [aux]
-        if kind is None or kind == COST_LOCAL_VECTOR or not type(self.loss).FUSED or self.flatten_dims:
+        if kind is None or kind in _NO_FUSED_ROBUST or not type(self.loss).FUSED or self.flatten_dims:
             return None, aux   # generic route (engine: torch.func Jacobians through generic_jacobians_error / generic_error)
         return kind, (aux if len(aux) > 1 else aux[0])
 

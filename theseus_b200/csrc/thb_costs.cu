@@ -33,6 +33,10 @@ template <typename T> struct GroupDev {
   int robust_kind;
   const T* const* log_radius;
   const int32_t* bstride_lr;
+  const T* const* x2;
+  const T* const* x3;
+  const int32_t* bstride3;
+  int sdf_rows, sdf_cols;
 };
 
 template <typename T> static GroupDev<T> to_dev(const thb_cost_group* g) {
@@ -57,6 +61,11 @@ template <typename T> static GroupDev<T> to_dev(const thb_cost_group* g) {
   d.robust_kind = g->robust_kind;
   d.log_radius = reinterpret_cast<const T* const*>(g->log_radius);
   d.bstride_lr = g->bstride_lr;
+  d.x2 = reinterpret_cast<const T* const*>(g->x2);
+  d.x3 = reinterpret_cast<const T* const*>(g->x3);
+  d.bstride3 = g->bstride3;
+  d.sdf_rows = g->sdf_rows;
+  d.sdf_cols = g->sdf_cols;
   return d;
 }
 
@@ -518,6 +527,285 @@ template <typename T> __global__ void error_reduce_kernel(const T* __restrict__ 
 }
 
 // ------------------------------------------------------------------------------------------------
+// 2-D motion planning (theseus/embodied/collision/collision.py, signed_distance_field.py:163-241,
+// theseus/embodied/motionmodel/double_integrator.py:16-175).
+
+// Collision2D: bilinear signed distance d of the pose's xy in the grid sdf_data [Bs, rows, cols] (cell (r, c) at
+// origin + (c, r) * cell_size; floor / ceil indices clamped, weights not; 0 and zero gradient outside the grid),
+// e = max(eps - d, 0) * w, J = -grad d (times [R 0] for SE2) * w, zeroed where d > eps.  DOF = 2 (Point2) or 3 (SE2).
+template <typename T, bool IS_SE2, bool WITH_J>
+__device__ __forceinline__ void collision2d_cost(const GroupDev<T>& g, int k, int64_t b, T w, T* e, T* J) {
+  const T* x = g.x0[k] + (int64_t)g.bstride[k * 4 + 0] * b;
+  const T* org = g.aux[k] + (int64_t)g.bstride[k * 4 + 2] * b;
+  const T* data = g.aux2[k] + (int64_t)g.bstride2[k * 3 + 0] * b;
+  const T cell = (g.aux3[k] + (int64_t)g.bstride2[k * 3 + 1] * b)[0];
+  const T eps = (g.aux4[k] + (int64_t)g.bstride2[k * 3 + 2] * b)[0];
+  const int rows = g.sdf_rows, cols = g.sdf_cols;
+  const T px = x[0], py = x[1], ox = org[0], oy = org[1];
+  const bool oob = (px < ox) || (px > ox + (T(cols) - T(1)) * cell) || (py < oy) || (py > oy + (T(rows) - T(1)) * cell);
+  const T col = (px - ox) / cell, row = (py - oy) / cell;
+  const T lr = floor(row), lc = floor(col);
+  const T hr = lr + T(1), hc = lc + T(1);
+  // float clamp first so that the integer conversion is defined for any input; the index clamp is the reference's
+  auto idx = [](T v, int n) -> int64_t {
+    const T vc = v < T(-1) ? T(-1) : (v > T(n) ? T(n) : v);
+    const int64_t i = (int64_t)vc;
+    return i < 0 ? 0 : (i > n - 1 ? n - 1 : i);
+  };
+  const int64_t lri = idx(lr, rows), hri = idx(hr, rows), lci = idx(lc, cols), hci = idx(hc, cols);
+  const T s_ll = data[lri * cols + lci], s_hl = data[hri * cols + lci], s_lh = data[lri * cols + hci], s_hh = data[hri * cols + hci];
+  const T hrd = hr - row, hcd = hc - col, lrd = row - lr, lcd = col - lc;
+  T dist = hrd * hcd * s_ll + lrd * hcd * s_hl + hrd * lcd * s_lh + lrd * lcd * s_hh;
+  if (oob) dist = T(0);
+  const T err = eps - dist;
+  e[0] = (err > T(0) ? err : T(0)) * w;
+  if (WITH_J) {
+    T gx = (hrd * (s_lh - s_ll) + lrd * (s_hh - s_hl)) / cell;
+    T gy = (hcd * (s_hl - s_ll) + lcd * (s_hh - s_lh)) / cell;
+    if (oob || dist > eps) { gx = T(0); gy = T(0); }
+    if (IS_SE2) {  // d xy / d tangent = [R 0] (SE2.xy Jacobian)
+      const T c = x[2], s = x[3];
+      J[0] = -(gx * c + gy * s) * w;
+      J[1] = -(-gx * s + gy * c) * w;
+      J[2] = T(0) * w;
+    } else {
+      J[0] = -gx * w;
+      J[1] = -gy * w;
+    }
+  }
+}
+
+template <typename T> __device__ __forceinline__ T weight_scalar(const GroupDev<T>& g, int k, int64_t b) {
+  return (g.w[k] + (int64_t)g.bstride[k * 4 + 3] * b)[0];
+}
+
+template <typename T, bool IS_SE2>
+__global__ void __launch_bounds__(128) linearize_collision2d_kernel(GroupDev<T> g, int64_t B, T* __restrict__ A_val, int64_t nnz,
+                                                                    T* __restrict__ bvec, int64_t m) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (int64_t)g.K * B) return;
+  const int k = (int)(t / B);
+  const int64_t b = t - (int64_t)k * B;
+  constexpr int DOF = IS_SE2 ? 3 : 2;
+  const T w = weight_scalar(g, k, b);      // dim 1: scale and diagonal weights are one value
+  T e[1], J[DOF];
+  if (w == T(0)) {
+    e[0] = T(0);
+#pragma unroll
+    for (int c = 0; c < DOF; c++) J[c] = T(0);
+  } else {
+    collision2d_cost<T, IS_SE2, true>(g, k, b, w, e, J);
+  }
+  T* Arow = A_val + b * nnz + g.a_off[k] + g.bp[k * 2 + 0];
+#pragma unroll
+  for (int c = 0; c < DOF; c++) Arow[c] = J[c];
+  bvec[b * m + g.row0[k]] = -e[0];
+}
+
+template <typename T, bool IS_SE2>
+__global__ void __launch_bounds__(128) error_collision2d_kernel(GroupDev<T> g, int64_t B, T* __restrict__ partial) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int nchunks = (g.K + kErrCostsPerThread - 1) / kErrCostsPerThread;
+  if (t >= (int64_t)nchunks * B) return;
+  const int c = (int)(t / B);
+  const int64_t b = t - (int64_t)c * B;
+  T acc = T(0);
+  const int k1 = min(g.K, (c + 1) * kErrCostsPerThread);
+  for (int k = c * kErrCostsPerThread; k < k1; k++) {
+    const T w = weight_scalar(g, k, b);
+    if (w == T(0)) continue;
+    T e[1];
+    collision2d_cost<T, IS_SE2, false>(g, k, b, w, e, nullptr);
+    acc += e[0] * e[0];
+  }
+  partial[(int64_t)c * B + b] = acc * T(0.5);
+}
+
+// Weight of a DOUBLE_INTEGRATOR cost function as a (2D x 2D) matrix Wm applied from the left (e <- Wm e, J <- Wm J):
+// scale / diagonal: diag(w); GP: U = (chol(M) (x) chol(Qc_inv^T))^T, U[(q,j),(p,i)] = Lm[p][q] Lq[i][j] (row (p,i) = p D + i).
+// Returns true if the weight is all zero (masked cost function, like load_weight).
+template <typename T, int D>
+__device__ __forceinline__ bool integrator_weight(const GroupDev<T>& g, int k, int64_t b, T* Wm) {
+  constexpr int N = 2 * D;
+#pragma unroll
+  for (int i = 0; i < N * N; i++) Wm[i] = T(0);
+  const T* wp = g.w[k] + (int64_t)g.bstride[k * 4 + 3] * b;
+  if (g.weight_kind == THB_WEIGHT_GP) {
+    const T dt = (g.aux2[k] + (int64_t)g.bstride2[k * 3 + 0] * b)[0];
+    const T idt = T(1) / dt;
+    const T lm00 = t_sqrt(T(12) * idt * idt * idt);
+    const T lm10 = (T(-6) * idt * idt) / lm00;
+    const T lm11 = t_sqrt(T(4) * idt - lm10 * lm10);
+    const T Lm[2][2] = {{lm00, T(0)}, {lm10, lm11}};
+    T Lq[D][D];
+#pragma unroll
+    for (int j = 0; j < D; j++) {
+      T s = wp[j * D + j];
+#pragma unroll
+      for (int q = 0; q < j; q++) s -= Lq[j][q] * Lq[j][q];
+      const T ljj = t_sqrt(s);
+      Lq[j][j] = ljj;
+#pragma unroll
+      for (int i = j + 1; i < D; i++) {
+        T a = wp[j * D + i];          // (Qc_inv^T)[i][j]
+#pragma unroll
+        for (int q = 0; q < j; q++) a -= Lq[i][q] * Lq[j][q];
+        Lq[i][j] = a / ljj;
+      }
+#pragma unroll
+      for (int i = 0; i < j; i++) Lq[i][j] = T(0);
+    }
+#pragma unroll
+    for (int p = 0; p < 2; p++)
+#pragma unroll
+      for (int q = 0; q < 2; q++)
+#pragma unroll
+        for (int i = 0; i < D; i++)
+#pragma unroll
+          for (int j = 0; j < D; j++) Wm[(q * D + j) * N + (p * D + i)] = Lm[p][q] * Lq[i][j];
+    return false;
+  }
+  bool all_zero = true;
+#pragma unroll
+  for (int r = 0; r < N; r++) {
+    const T v = (g.weight_kind == THB_WEIGHT_SCALE) ? wp[0] : wp[r];
+    Wm[r * N + r] = v;
+    all_zero = all_zero && (v == T(0));
+  }
+  return all_zero;
+}
+
+// Unweighted error [2D] and the pose Jacobians (top D x D blocks; the rest of the four blocks is constant) of
+// e = [pose1.local(pose2) - dt vel1 ; vel2 - vel1].  SE2: local = log(pose1^-1 pose2), J1 = -dlog Ad(D^-1), J2 = dlog
+// (= Between with an identity measurement); Vector: local = pose2 - pose1, J1 = -I, J2 = I.
+template <typename T, int D, bool IS_SE2, bool WITH_J>
+__device__ __forceinline__ T integrator_error(const GroupDev<T>& g, int k, int64_t b, T* e, T* Jp1, T* Jp2) {
+  const T* p1 = g.x0[k] + (int64_t)g.bstride[k * 4 + 0] * b;
+  const T* v1 = g.x1[k] + (int64_t)g.bstride[k * 4 + 1] * b;
+  const T* p2 = g.x2[k] + (int64_t)g.bstride3[k * 2 + 0] * b;
+  const T* v2 = g.x3[k] + (int64_t)g.bstride3[k * 2 + 1] * b;
+  const T dt = (g.aux[k] + (int64_t)g.bstride[k * 4 + 2] * b)[0];
+  T loc[D];
+  if (IS_SE2) {
+    T X0[4], X1[4], Dm[4], Jl[9];
+    load_n<T, 4>(p1, X0);
+    load_n<T, 4>(p2, X1);
+    se2_between(X0, X1, Dm);
+    se2_log_jlog<T, WITH_J>(Dm, loc, Jl);
+    if (WITH_J) {
+      T Di[4], Ad[9];
+      se2_inverse(Dm, Di);
+      se2_adjoint(Di, Ad);
+#pragma unroll
+      for (int r = 0; r < 3; r++)
+#pragma unroll
+        for (int c = 0; c < 3; c++) {
+          Jp1[r * D + c] = -(Jl[r * 3 + 0] * Ad[0 * 3 + c] + Jl[r * 3 + 1] * Ad[1 * 3 + c] + Jl[r * 3 + 2] * Ad[2 * 3 + c]);
+          Jp2[r * D + c] = Jl[r * 3 + c];
+        }
+    }
+  } else {
+#pragma unroll
+    for (int i = 0; i < D; i++) loc[i] = p2[i] - p1[i];
+    if (WITH_J) {
+#pragma unroll
+      for (int r = 0; r < D; r++)
+#pragma unroll
+        for (int c = 0; c < D; c++) {
+          Jp1[r * D + c] = (r == c) ? T(-1) : T(0);
+          Jp2[r * D + c] = (r == c) ? T(1) : T(0);
+        }
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < D; i++) {
+    const T a = v1[i];
+    e[i] = loc[i] - dt * a;
+    e[D + i] = v2[i] - a;
+  }
+  return dt;
+}
+
+template <typename T, int D, bool IS_SE2>
+__global__ void __launch_bounds__(128) linearize_integrator_kernel(GroupDev<T> g, int64_t B, T* __restrict__ A_val, int64_t nnz,
+                                                                   T* __restrict__ bvec, int64_t m) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (int64_t)g.K * B) return;
+  const int k = (int)(t / B);
+  const int64_t b = t - (int64_t)k * B;
+  constexpr int N = 2 * D;
+  T Wm[N * N], e[N], Jp1[D * D], Jp2[D * D];
+  const bool masked = integrator_weight<T, D>(g, k, b, Wm);
+  const T dt = integrator_error<T, D, IS_SE2, true>(g, k, b, e, Jp1, Jp2);
+  T* Arow = A_val + b * nnz + g.a_off[k];
+  const int stride = g.a_stride[k];
+  const int bp0 = g.bp[k * 4 + 0], bp1 = g.bp[k * 4 + 1], bp2 = g.bp[k * 4 + 2], bp3 = g.bp[k * 4 + 3];
+  T* brow = bvec + b * m + g.row0[k];
+  // unweighted blocks, column c of variable slot: pose1 [Jp1; 0], vel1 [-dt I; -I], pose2 [Jp2; 0], vel2 [0; I]
+#pragma unroll
+  for (int r = 0; r < N; r++) {
+    T o0[D], o1[D], o2[D], o3[D];
+    T we = T(0);
+#pragma unroll
+    for (int c = 0; c < D; c++) { o0[c] = T(0); o1[c] = T(0); o2[c] = T(0); o3[c] = T(0); }
+#pragma unroll
+    for (int q = 0; q < N; q++) {
+      const T wq = Wm[r * N + q];
+      we += wq * e[q];
+      if (q < D) {
+#pragma unroll
+        for (int c = 0; c < D; c++) {
+          o0[c] += wq * Jp1[q * D + c];
+          o2[c] += wq * Jp2[q * D + c];
+        }
+        o1[q] += wq * (-dt);
+      } else {
+        o1[q - D] -= wq;
+        o3[q - D] += wq;
+      }
+    }
+    if (masked) {
+      we = T(0);
+#pragma unroll
+      for (int c = 0; c < D; c++) { o0[c] = T(0); o1[c] = T(0); o2[c] = T(0); o3[c] = T(0); }
+    }
+#pragma unroll
+    for (int c = 0; c < D; c++) {
+      Arow[r * stride + bp0 + c] = o0[c];
+      Arow[r * stride + bp1 + c] = o1[c];
+      Arow[r * stride + bp2 + c] = o2[c];
+      Arow[r * stride + bp3 + c] = o3[c];
+    }
+    brow[r] = -we;
+  }
+}
+
+template <typename T, int D, bool IS_SE2>
+__global__ void __launch_bounds__(128) error_integrator_kernel(GroupDev<T> g, int64_t B, T* __restrict__ partial) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int nchunks = (g.K + kErrCostsPerThread - 1) / kErrCostsPerThread;
+  if (t >= (int64_t)nchunks * B) return;
+  const int c = (int)(t / B);
+  const int64_t b = t - (int64_t)c * B;
+  constexpr int N = 2 * D;
+  T acc = T(0);
+  const int k1 = min(g.K, (c + 1) * kErrCostsPerThread);
+  for (int k = c * kErrCostsPerThread; k < k1; k++) {
+    T Wm[N * N], e[N];
+    if (integrator_weight<T, D>(g, k, b, Wm)) continue;
+    integrator_error<T, D, IS_SE2, false>(g, k, b, e, nullptr, nullptr);
+#pragma unroll
+    for (int r = 0; r < N; r++) {
+      T we = T(0);
+#pragma unroll
+      for (int q = 0; q < N; q++) we += Wm[r * N + q] * e[q];
+      acc += we * we;
+    }
+  }
+  partial[(int64_t)c * B + b] = acc * T(0.5);
+}
+
+// ------------------------------------------------------------------------------------------------
 template <typename T> struct VarDev {
   int N;
   const T* const* x;
@@ -733,6 +1021,26 @@ template <typename T> __global__ void k_se3_compose(const T* __restrict__ G0, co
 // ------------------------------------------------------------------------------------------------
 static inline unsigned grid_for(int64_t total, int threads) { return (unsigned)((total + threads - 1) / threads); }
 
+// Argument checks of the motion-planning kinds: which tables must be present, which weights each kind takes.
+static int check_collision2d(const thb_cost_group* g) {
+  if (g->aux2 == nullptr || g->aux3 == nullptr || g->aux4 == nullptr || g->bstride2 == nullptr) return THB_ERR_BAD_ARG;
+  if (g->sdf_rows < 1 || g->sdf_cols < 1 || g->dim != 1) return THB_ERR_BAD_ARG;
+  if (g->weight_kind != THB_WEIGHT_SCALE && g->weight_kind != THB_WEIGHT_DIAGONAL) return THB_ERR_UNSUPPORTED;
+  if (g->robust_kind != THB_ROBUST_NONE) return THB_ERR_UNSUPPORTED;
+  return THB_OK;
+}
+static int check_integrator(const thb_cost_group* g) {
+  if (g->x2 == nullptr || g->x3 == nullptr || g->bstride3 == nullptr) return THB_ERR_BAD_ARG;
+  if (g->kind == THB_COST_DOUBLE_INTEGRATOR_SE2 ? g->dim != 6 : (g->dim != 4 && g->dim != 6)) return THB_ERR_BAD_ARG;
+  if (g->weight_kind == THB_WEIGHT_GP) {
+    if (g->aux2 == nullptr || g->bstride2 == nullptr) return THB_ERR_BAD_ARG;
+  } else if (g->weight_kind != THB_WEIGHT_SCALE && g->weight_kind != THB_WEIGHT_DIAGONAL) {
+    return THB_ERR_UNSUPPORTED;
+  }
+  if (g->robust_kind != THB_ROBUST_NONE) return THB_ERR_UNSUPPORTED;
+  return THB_OK;
+}
+
 template <typename T>
 static int linearize_group(const thb_cost_group* g, int64_t B, T* A_val, int64_t nnz, T* b, int64_t m, thb_stream_t s) {
   if (g == nullptr || g->K < 0 || B < 0) return THB_ERR_BAD_ARG;
@@ -763,6 +1071,23 @@ static int linearize_group(const thb_cost_group* g, int64_t B, T* A_val, int64_t
       if (g->aux2 == nullptr || g->aux3 == nullptr || g->aux4 == nullptr || g->bstride2 == nullptr) return THB_ERR_BAD_ARG;
       linearize_reprojection_kernel<T><<<grid, 128, 0, cs>>>(d, B, A_val, nnz, b, m);
       break;
+    case THB_COST_COLLISION2D_POINT2:
+    case THB_COST_COLLISION2D_SE2: {
+      const int rc = check_collision2d(g);
+      if (rc != THB_OK) return rc;
+      if (g->kind == THB_COST_COLLISION2D_SE2) linearize_collision2d_kernel<T, true><<<grid, 128, 0, cs>>>(d, B, A_val, nnz, b, m);
+      else linearize_collision2d_kernel<T, false><<<grid, 128, 0, cs>>>(d, B, A_val, nnz, b, m);
+      break;
+    }
+    case THB_COST_DOUBLE_INTEGRATOR_VECTOR:
+    case THB_COST_DOUBLE_INTEGRATOR_SE2: {
+      const int rc = check_integrator(g);
+      if (rc != THB_OK) return rc;
+      if (g->kind == THB_COST_DOUBLE_INTEGRATOR_SE2) linearize_integrator_kernel<T, 3, true><<<grid, 128, 0, cs>>>(d, B, A_val, nnz, b, m);
+      else if (g->dim == 4) linearize_integrator_kernel<T, 2, false><<<grid, 128, 0, cs>>>(d, B, A_val, nnz, b, m);
+      else linearize_integrator_kernel<T, 3, false><<<grid, 128, 0, cs>>>(d, B, A_val, nnz, b, m);
+      break;
+    }
     default: return THB_ERR_UNSUPPORTED;
   }
   THB_CHECK_LAUNCH();
@@ -788,6 +1113,23 @@ template <typename T> static int error_group(const thb_cost_group* g, int64_t B,
       if (g->aux2 == nullptr || g->aux3 == nullptr || g->aux4 == nullptr || g->bstride2 == nullptr) return THB_ERR_BAD_ARG;
       error_reprojection_kernel<T><<<grid, 128, 0, cs>>>(d, B, partial);
       break;
+    case THB_COST_COLLISION2D_POINT2:
+    case THB_COST_COLLISION2D_SE2: {
+      const int rc = check_collision2d(g);
+      if (rc != THB_OK) return rc;
+      if (g->kind == THB_COST_COLLISION2D_SE2) error_collision2d_kernel<T, true><<<grid, 128, 0, cs>>>(d, B, partial);
+      else error_collision2d_kernel<T, false><<<grid, 128, 0, cs>>>(d, B, partial);
+      break;
+    }
+    case THB_COST_DOUBLE_INTEGRATOR_VECTOR:
+    case THB_COST_DOUBLE_INTEGRATOR_SE2: {
+      const int rc = check_integrator(g);
+      if (rc != THB_OK) return rc;
+      if (g->kind == THB_COST_DOUBLE_INTEGRATOR_SE2) error_integrator_kernel<T, 3, true><<<grid, 128, 0, cs>>>(d, B, partial);
+      else if (g->dim == 4) error_integrator_kernel<T, 2, false><<<grid, 128, 0, cs>>>(d, B, partial);
+      else error_integrator_kernel<T, 3, false><<<grid, 128, 0, cs>>>(d, B, partial);
+      break;
+    }
     default: return THB_ERR_UNSUPPORTED;
   }
   THB_CHECK_LAUNCH();

@@ -1,9 +1,310 @@
-"""`th.eb` namespace of the reference (theseus/embodied/__init__.py): Between / Local / Reprojection have fused CUDA schemas;
-MovingFrameBetween runs on the torch path (torch.func Jacobians + tangent-space projection, like an AutoDiffCostFunction)."""
-from typing import Optional
+"""`th.eb` namespace of the reference (theseus/embodied/__init__.py): Between / Local / Reprojection and the 2-D motion-planning costs
+(Collision2D, DoubleIntegrator / GPMotionModel with GPCostWeight) have fused CUDA schemas; MovingFrameBetween and the tactile costs run
+on the torch path (torch.func Jacobians + tangent-space projection, like an AutoDiffCostFunction)."""
+from typing import List, Optional, Tuple, Union
 
-from .core import Between, CostFunction, CostWeight, Difference, Local, Reprojection  # noqa: F401
-from .geometry import LieGroup
+import torch
+
+from .core import (COST_COLLISION2D_POINT2, COST_COLLISION2D_SE2, COST_DOUBLE_INTEGRATOR_SE2, COST_DOUBLE_INTEGRATOR_VECTOR,  # noqa: F401
+                   WEIGHT_GP, Between, CostFunction, CostWeight, Difference, Local, Reprojection)
+from .geometry import SE2, LieGroup, Point2, Variable, Vector, as_variable
+
+
+def _bilinear_sdf(data, ox, oy, cell, px, py):
+    """Bilinear lookup of signed_distance_field.py:163-241: grid data [Bs, rows, cols], cell (r, c) at (ox, oy) + (c, r) * cell;
+    floor / ceil indices clamped to the grid, the interpolation weights not; 0 outside [ox, ox + (cols-1) cell] x [oy, ...].
+    px, py [B, ...] (the batch index of `data` is broadcast over the trailing dimensions); ox, oy, cell broadcast against them.
+    Returns (dist, d dist / d px, d dist / d py) -- the gradient is 0 outside the grid, like the reference's."""
+    nrows, ncols = data.shape[-2], data.shape[-1]
+    oob = (px < ox) | (px > ox + (ncols - 1.0) * cell) | (py < oy) | (py > oy + (nrows - 1.0) * cell)
+    col, row = (px - ox) / cell, (py - oy) / cell
+    lr, lc = torch.floor(row), torch.floor(col)
+    hr, hc = lr + 1.0, lc + 1.0
+    lri, lci = lr.long().clamp(0, nrows - 1), lc.long().clamp(0, ncols - 1)
+    hri, hci = hr.long().clamp(0, nrows - 1), hc.long().clamp(0, ncols - 1)
+    bi = torch.arange(data.shape[0], device=data.device).view((-1,) + (1,) * (px.ndim - 1))
+    g = lambda r, c: data[bi, r, c]
+    s_ll, s_hl, s_lh, s_hh = g(lri, lci), g(hri, lci), g(lri, hci), g(hri, hci)
+    dist = (hr - row) * (hc - col) * s_ll + (row - lr) * (hc - col) * s_hl + (hr - row) * (col - lc) * s_lh + (row - lr) * (col - lc) * s_hh
+    dist = torch.where(oob, torch.zeros_like(dist), dist)    # sdf_boundary_value = 0 (signed_distance_field.py:26)
+    jx = ((hr - row) * (s_lh - s_ll) + (row - lr) * (s_hh - s_hl)) / cell
+    jy = ((hc - col) * (s_hl - s_ll) + (col - lc) * (s_hh - s_lh)) / cell
+    zero = torch.zeros_like(jx)
+    return dist, torch.where(oob, zero, jx), torch.where(oob, zero, jy)
+
+
+class SignedDistanceField2D:
+    """theseus/embodied/collision/signed_distance_field.py:16-246: a batch of 2-D signed distance grids sdf_data [Bs, rows, cols] with
+    origin [Bo, 2] (cell (r, c) at origin + (c, r) * cell_size) and cell_size [Bc, 1]; bilinear interpolation, 0 outside the grid."""
+
+    def __init__(self, origin: Union[Point2, torch.Tensor], cell_size: Union[float, torch.Tensor, Variable],
+                 sdf_data: Optional[Union[torch.Tensor, Variable]] = None, occupancy_map: Optional[Union[torch.Tensor, Variable]] = None,
+                 occupancy_threshold: float = 0.75, sdf_boundary_value: float = 0.0):
+        if occupancy_map is not None:
+            if sdf_data is not None:
+                raise ValueError("Only one of sdf_data and occupancy_map should be provided.")
+            sdf_data = self._compute_sdf_data_from_map(occupancy_map, SignedDistanceField2D.convert_cell_size(cell_size).tensor,
+                                                       threshold=occupancy_threshold)
+        elif sdf_data is None:
+            raise ValueError("Either sdf_data or argument occupancy_map should be provided.")
+        self.update_data(origin, sdf_data, cell_size)
+        self._num_rows = sdf_data.shape[1]
+        self._num_cols = sdf_data.shape[2]
+        self.sdf_boundary_value = sdf_boundary_value
+
+    def _compute_sdf_data_from_map(self, occupancy_map_batch, cell_size: torch.Tensor, threshold: float = 0.75) -> Variable:
+        """signed_distance_field.py:54-100 (gpmp2's map -> SDF: Euclidean distance transforms of the map and of its complement)."""
+        from scipy import ndimage
+        if isinstance(occupancy_map_batch, Variable):
+            occupancy_map_batch = occupancy_map_batch.tensor
+        if cell_size.shape[0] != occupancy_map_batch.shape[0]:
+            cell_size = cell_size.expand(occupancy_map_batch.shape[0], 1)
+        if occupancy_map_batch.ndim != 3:
+            raise ValueError("Argument occupancy_map to SignedDistanceField2D must be a batch of matrices.")
+        out = []
+        for i in range(occupancy_map_batch.shape[0]):
+            occupancy_map = occupancy_map_batch[i]
+            cur_map = (occupancy_map > threshold).int()
+            if torch.max(cur_map) == 0:
+                max_map_size = 2 * cell_size[i].item() * max(occupancy_map.size(0), occupancy_map.size(1))
+                sdf = torch.ones(occupancy_map.shape, dtype=occupancy_map.dtype) * max_map_size
+            else:
+                map_dist = ndimage.distance_transform_edt((1 - cur_map).cpu().numpy())
+                inv_map_dist = ndimage.distance_transform_edt(cur_map.cpu().numpy())
+                sdf = torch.tensor(map_dist - inv_map_dist, dtype=occupancy_map.dtype) * cell_size[i].cpu()
+            out.append(sdf)
+        return Variable(torch.stack(out))
+
+    @staticmethod
+    def convert_origin(origin: Union[torch.Tensor, Point2]) -> Point2:
+        if not isinstance(origin, (Point2, torch.Tensor)):
+            raise ValueError("Argument origin to SignedDistanceField2D must be either a tensor or a Point2 variable.")
+        if not isinstance(origin, Point2):
+            try:
+                return Point2(tensor=origin)
+            except ValueError:
+                raise ValueError("Argument origin to SignedDistanceField2D must be a batch of 2D tensors.")
+        return origin
+
+    @staticmethod
+    def convert_cell_size(cell_size: Union[float, torch.Tensor, Variable]) -> Variable:
+        if not isinstance(cell_size, Variable):
+            if not isinstance(cell_size, torch.Tensor):
+                if not isinstance(cell_size, float):
+                    raise ValueError("Argument cell_size must be either a Variable, tensor, or float.")
+                cell_size = torch.tensor(cell_size).view(-1, 1)
+            return Variable(cell_size)
+        if not (cell_size.ndim == 1 or (cell_size.ndim == 2 and cell_size.shape[1] == 1)):
+            raise ValueError("Argument cell_size must be a batch of 0D or 1D tensors.")
+        return cell_size
+
+    @staticmethod
+    def convert_sdf_data(sdf_data: Union[torch.Tensor, Variable]) -> Variable:
+        sdf_data = as_variable(sdf_data)
+        if sdf_data.ndim != 3:
+            raise ValueError("Argument sdf_data to SignedDistanceField2D must be a batch of matrices.")
+        return sdf_data
+
+    def update_data(self, origin, sdf_data, cell_size):
+        self.origin = SignedDistanceField2D.convert_origin(origin)
+        self.cell_size = SignedDistanceField2D.convert_cell_size(cell_size)
+        self.sdf_data = SignedDistanceField2D.convert_sdf_data(sdf_data)
+
+    def convert_points_to_cell(self, points: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """points [B, 2, N] -> (row, col, out_of_bounds), each [B, N]."""
+        origin = self.origin.tensor.unsqueeze(-1) if self.origin.ndim == 2 else self.origin.tensor
+        cell_size = self.cell_size.tensor if self.cell_size.ndim == 2 else self.cell_size.tensor.unsqueeze(-1)
+        px, py = points[:, 0], points[:, 1]
+        oob = ((px < origin[:, 0]) | (px > origin[:, 0] + (self._num_cols - 1.0) * cell_size)
+               | (py < origin[:, 1]) | (py > origin[:, 1] + (self._num_rows - 1.0) * cell_size))
+        return (py - origin[:, 1]) / cell_size, (px - origin[:, 0]) / cell_size, oob
+
+    def signed_distance(self, points: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+        """points [B, 2, N] -> (distances [B, N], Jacobians d dist / d point [B, N, 2])."""
+        origin = self.origin.tensor
+        cell = self.cell_size.tensor if self.cell_size.ndim == 2 else self.cell_size.tensor.unsqueeze(-1)
+        data = self.sdf_data.tensor
+        px, py = points[:, 0], points[:, 1]
+        B = max(px.shape[0], data.shape[0])
+        if data.shape[0] != B:
+            data = data.expand(B, -1, -1)
+        px, py = px.expand(B, -1), py.expand(B, -1)
+        dist, jx, jy = _bilinear_sdf(data, origin[:, 0:1], origin[:, 1:2], cell, px, py)
+        if self.sdf_boundary_value != 0.0:
+            _, _, oob = self.convert_points_to_cell(points.expand(B, -1, -1))
+            dist = torch.where(oob, torch.full_like(dist, self.sdf_boundary_value), dist)
+        return dist, torch.stack([jx, jy], dim=2)
+
+    def to(self, *args, **kwargs):
+        self.cell_size.to(*args, **kwargs)
+        self.origin.to(*args, **kwargs)
+        self.sdf_data.to(*args, **kwargs)
+
+
+class Collision2D(CostFunction):
+    """theseus/embodied/collision/collision.py:17-110: e = max(cost_eps - sdf(pose.xy), 0), dim 1; J = -grad sdf (times the SE2.xy
+    Jacobian [R 0] for SE2 poses), zero where sdf > cost_eps.  Fused kernels THB_COST_COLLISION2D_POINT2 / _SE2 (thb_costs.cu)."""
+
+    def __init__(self, pose: Union[Point2, SE2], sdf_origin: Union[Point2, torch.Tensor], sdf_data: Union[torch.Tensor, Variable],
+                 sdf_cell_size: Union[float, torch.Tensor, Variable], cost_eps: Union[float, Variable, torch.Tensor],
+                 cost_weight: CostWeight, name: Optional[str] = None):
+        if not isinstance(pose, (Point2, SE2)):
+            raise ValueError("Collision2D only accepts Point2 or SE2 poses.")
+        super().__init__(cost_weight, name=name)
+        self.pose = pose
+        self.sdf_origin = SignedDistanceField2D.convert_origin(sdf_origin)
+        self.sdf_data = SignedDistanceField2D.convert_sdf_data(sdf_data)
+        self.sdf_cell_size = SignedDistanceField2D.convert_cell_size(sdf_cell_size)
+        self.cost_eps = as_variable(cost_eps)
+        self.cost_eps.tensor = self.cost_eps.tensor.view(-1, 1)
+        self.register_optim_vars(["pose"])
+        self.register_aux_vars(["sdf_origin", "sdf_data", "sdf_cell_size", "cost_eps"])
+        self.sdf = SignedDistanceField2D(self.sdf_origin, self.sdf_cell_size, self.sdf_data)
+
+    def dim(self) -> int:
+        return 1
+
+    def _torch_error(self, optim_tensors, aux_tensors):
+        x = optim_tensors[0]
+        origin, data, cell, eps = aux_tensors
+        dist, _, _ = _bilinear_sdf(data, origin[..., 0], origin[..., 1], cell.view(-1), x[..., 0], x[..., 1])
+        return (eps.view(-1) - dist).clamp(min=0).unsqueeze(-1)    # clamp's gradient is kept at dist == eps, like the reference
+
+    def schema(self):
+        return (COST_COLLISION2D_SE2 if isinstance(self.pose, SE2) else COST_COLLISION2D_POINT2,
+                [self.sdf_origin, self.sdf_data, self.sdf_cell_size, self.cost_eps])
+
+    def _copy_impl(self, new_name: Optional[str] = None) -> "Collision2D":
+        return Collision2D(self.pose.copy(), self.sdf_origin.copy(), self.sdf_data.copy(), self.sdf_cell_size.copy(),
+                           self.cost_eps.copy(), self.weight.copy(), name=new_name)
+
+    def set_aux_var_at(self, index: int, variable: Variable):
+        """Keeps the SDF container on the new auxiliary variable (collision.py:104-107)."""
+        super().set_aux_var_at(index, variable)
+        self.sdf.update_data(self.sdf_origin, self.sdf_data, self.sdf_cell_size)
+
+
+class DoubleIntegrator(CostFunction):
+    """theseus/embodied/motionmodel/double_integrator.py:16-95: e = [pose1.local(pose2) - dt vel1 ; vel2 - vel1], dim 2 dof.
+    Fused kernels for poses of Vector kind with dof 2 / 3 (THB_COST_DOUBLE_INTEGRATOR_VECTOR) and SE2 (_SE2); other poses take the
+    generic route on the same torch restatement."""
+
+    def __init__(self, pose1: LieGroup, vel1: Vector, pose2: LieGroup, vel2: Vector, dt: Union[float, torch.Tensor, Variable],
+                 cost_weight: CostWeight, name: Optional[str] = None):
+        super().__init__(cost_weight, name=name)
+        dof = pose1.dof()
+        if not (vel1.dof() == pose2.dof() == vel2.dof() == dof):
+            raise ValueError("All variables for a DoubleIntegrator must have the same dimension.")
+        self.dt = as_variable(dt)
+        if self.dt.tensor.squeeze().ndim > 1:
+            raise ValueError("dt data must be a 0-D or 1-D tensor with numel in {1, batch_size}.")
+        self.dt.tensor = self.dt.tensor.view(-1, 1)
+        self.pose1, self.vel1, self.pose2, self.vel2 = pose1, vel1, pose2, vel2
+        self.register_optim_vars(["pose1", "vel1", "pose2", "vel2"])
+        self.register_aux_vars(["dt"])
+
+    def dim(self) -> int:
+        return 2 * self.pose1.dof()
+
+    def _torch_error(self, optim_tensors, aux_tensors):
+        from . import lie_torch
+        p1, v1, p2, v2 = optim_tensors
+        dt = aux_tensors[0]
+        local = lie_torch.local(self.pose1.KIND, p1, p2)
+        return torch.cat([local - dt.view(-1, 1) * v1, v2 - v1], dim=-1)
+
+    def schema(self):
+        aux = [self.dt] + ([self.weight.dt] if getattr(self.weight, "WEIGHT_KIND", -1) == WEIGHT_GP else [])
+        vels_ok = isinstance(self.vel1, Vector) and isinstance(self.vel2, Vector)
+        same = type(self.pose1) is type(self.pose2)
+        if vels_ok and same and isinstance(self.pose1, SE2):
+            kind = COST_DOUBLE_INTEGRATOR_SE2
+        elif vels_ok and same and isinstance(self.pose1, Vector) and self.pose1.dof() in (2, 3):
+            kind = COST_DOUBLE_INTEGRATOR_VECTOR
+        else:
+            return None, aux                       # generic route
+        if aux[1:] and self.weight.Qc_inv.tensor.shape[-1] != self.pose1.dof():
+            return None, aux                       # (mismatched Qc_inv: the torch route raises the reference's shape error)
+        return kind, aux
+
+    def _copy_impl(self, new_name: Optional[str] = None) -> "DoubleIntegrator":
+        return type(self)(self.pose1.copy(), self.vel1.copy(), self.pose2.copy(), self.vel2.copy(), self.dt.copy(), self.weight.copy(),
+                          name=new_name)
+
+
+class GPCostWeight(CostWeight):
+    """theseus/embodied/motionmodel/double_integrator.py:98-175: the full-matrix weight of a constant-velocity Gaussian-process prior,
+    U = chol(W^T)^T with W = [[12/dt^3, -6/dt^2], [-6/dt^2, 4/dt]] (x) Qc_inv; weighting is U e, U J_i.  Qc_inv [d, d] or [Bq, d, d],
+    dt [Bw, 1].  On the DoubleIntegrator kinds the kernels form U in registers (THB_WEIGHT_GP); elsewhere the torch form below."""
+    WEIGHT_KIND = WEIGHT_GP
+
+    def __init__(self, Qc_inv: Union[Variable, torch.Tensor], dt: Union[float, Variable, torch.Tensor], name: Optional[str] = None):
+        super().__init__(name=name)
+        dt = as_variable(dt)
+        if dt.tensor.squeeze().ndim > 1:
+            raise ValueError("dt must be a 0-D or 1-D tensor.")
+        self.dt = dt
+        self.dt.tensor = self.dt.tensor.view(-1, 1)
+        if not (self.dt.tensor > 0).all():
+            raise ValueError("dt must be greater than 0.")
+        Qc_inv = as_variable(Qc_inv)
+        if Qc_inv.ndim not in [2, 3]:
+            raise ValueError("Qc_inv must be a single matrix or a batch of matrices.")
+        if not Qc_inv.shape[-2] == Qc_inv.shape[-1]:
+            raise ValueError("Qc_inv must contain square matrices.")
+        self.Qc_inv = Qc_inv
+        self.Qc_inv.tensor = Qc_inv.tensor if Qc_inv.ndim == 3 else Qc_inv.tensor.unsqueeze(0)
+        try:
+            torch.linalg.cholesky(Qc_inv.tensor)
+        except RuntimeError:
+            raise ValueError("Qc_inv must be positive definite.")
+        if self.dt.tensor.dtype != self.Qc_inv.tensor.dtype:
+            self.dt.tensor = self.dt.tensor.to(self.Qc_inv.tensor.dtype)
+        self.register_aux_vars(["Qc_inv", "dt"])
+
+    @property
+    def aux_vars(self) -> List[Variable]:
+        return [self.Qc_inv, self.dt]
+
+    def weight_tensor(self) -> Variable:
+        return self.Qc_inv
+
+    def is_zero(self) -> torch.Tensor:
+        return torch.zeros(self.Qc_inv.shape[0]).bool()
+
+    def _compute_cost_weight(self) -> torch.Tensor:
+        Q = self.Qc_inv.tensor
+        dof = Q.shape[-1]
+        dt = self.dt.tensor.view(-1, 1, 1)
+        q11, q12, q22 = 12.0 * dt.pow(-3.0) * Q, -6.0 * dt.pow(-2.0) * Q, 4.0 * dt.reciprocal() * Q
+        W = torch.cat([torch.cat([q11, q12], dim=-1), torch.cat([q12, q22], dim=-1)], dim=-2)
+        assert W.shape[-1] == 2 * dof
+        return torch.linalg.cholesky(W.transpose(-2, -1)).transpose(-2, -1)
+
+    def weight_error(self, error: torch.Tensor) -> torch.Tensor:
+        return torch.matmul(self._compute_cost_weight(), error.unsqueeze(2)).squeeze(2)
+
+    def weight_jacobians_and_error(self, jacobians, error):
+        U = self._compute_cost_weight()
+        return [torch.matmul(U, J) for J in jacobians], torch.matmul(U, error.unsqueeze(2)).squeeze(2)
+
+    def copy(self, new_name: Optional[str] = None, keep_variable_names: bool = False) -> "GPCostWeight":
+        return GPCostWeight(self.Qc_inv.copy(new_name=self.Qc_inv.name if keep_variable_names else None),
+                            self.dt.copy(new_name=self.dt.name if keep_variable_names else None), name=new_name)
+
+
+class GPMotionModel(DoubleIntegrator):
+    """double_integrator.py:178-207: a DoubleIntegrator whose weight must be a GPCostWeight."""
+
+    def __init__(self, pose1: LieGroup, vel1: Vector, pose2: LieGroup, vel2: Vector, dt: Union[float, Variable, torch.Tensor],
+                 cost_weight: GPCostWeight, name: Optional[str] = None):
+        if not isinstance(cost_weight, GPCostWeight):
+            raise ValueError("GPMotionModel only accepts cost weights of type GPCostWeight. "
+                             "For other weight types, consider using DoubleIntegrator instead.")
+        dt = as_variable(dt)
+        if dt.tensor.squeeze().ndim > 1:
+            raise ValueError("dt must be a 0-D or 1-D tensor.")
+        super().__init__(pose1, vel1, pose2, vel2, dt, cost_weight, name=name)
 
 
 class MovingFrameBetween(CostFunction):
@@ -158,25 +459,13 @@ class EffectorObjectContactPlanar(CostFunction):
         return 1
 
     def _torch_error(self, optim_tensors, aux_tensors):
-        import torch
         o, e = optim_tensors
         origin, data, cell, radius = aux_tensors
         cell, radius = cell.view(-1), radius.view(-1)
         dx, dy = e[..., 0] - o[..., 0], e[..., 1] - o[..., 1]
         px = o[..., 2] * dx + o[..., 3] * dy       # eff position in the object frame (SE2.transform_to)
         py = -o[..., 3] * dx + o[..., 2] * dy
-        nrows, ncols = data.shape[-2], data.shape[-1]
-        oob = (px < origin[..., 0]) | (px > origin[..., 0] + (ncols - 1.0) * cell) | (py < origin[..., 1]) | (py > origin[..., 1] + (nrows - 1.0) * cell)
-        col, row = (px - origin[..., 0]) / cell, (py - origin[..., 1]) / cell
-        lr, lc = torch.floor(row), torch.floor(col)
-        hr, hc = lr + 1.0, lc + 1.0
-        lri, lci = lr.long().clamp(0, nrows - 1), lc.long().clamp(0, ncols - 1)
-        hri, hci = hr.long().clamp(0, nrows - 1), hc.long().clamp(0, ncols - 1)
-        bi = torch.arange(data.shape[0], device=data.device)
-        g = lambda r, c: data[bi, r, c]
-        dist = (hr - row) * (hc - col) * g(lri, lci) + (row - lr) * (hc - col) * g(hri, lci) \
-            + (hr - row) * (col - lc) * g(lri, hci) + (row - lr) * (col - lc) * g(hri, hci)
-        dist = torch.where(oob, torch.zeros_like(dist), dist)    # sdf_boundary_value = 0 (signed_distance_field.py:26)
+        dist, _, _ = _bilinear_sdf(data, origin[..., 0], origin[..., 1], cell, px, py)
         return (dist - radius).abs().unsqueeze(-1)
 
     def schema(self):

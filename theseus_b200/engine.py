@@ -33,6 +33,19 @@ def _batched_torch_route() -> bool:
     return os.environ.get("THB_BATCHED_TORCH_ROUTE", "0") == "1"
 
 
+# cost kinds with four optimisation variables (thb_cost_group.x2 / x3, bp of width 4) and the weight kinds each kernel takes
+_FOUR_VAR_KINDS = (10, 11)             # THB_COST_DOUBLE_INTEGRATOR_VECTOR / _SE2
+_COLLISION_KINDS = (8, 9)              # THB_COST_COLLISION2D_POINT2 / _SE2
+_WEIGHT_SCALE, _WEIGHT_DIAGONAL, _WEIGHT_GP = 0, 1, 2
+
+
+def _fused_weight(kind: int, weight_kind: int) -> bool:
+    """True if the linearize / error kernels of `kind` apply cost weights of `weight_kind` (include/thb200.h, enum thb_weight_kind)."""
+    if weight_kind in (_WEIGHT_SCALE, _WEIGHT_DIAGONAL):
+        return True
+    return weight_kind == _WEIGHT_GP and kind in _FOUR_VAR_KINDS
+
+
 def _require_cuda_device(device):
     """The product has no CPU path: fail loudly.  (tests/test_simt_engine_emulation.py replaces this guard AND the library by a host
     emulation of the kernels to exercise the host code without a GPU; nothing in the package does.)"""
@@ -89,18 +102,19 @@ class Engine:
         for f, cf in enumerate(costs):
             kind, aux = cf.schema()
             self._aux_of.append(list(aux) if isinstance(aux, (list, tuple)) else [aux])
-            if kind is None or cf.weight.WEIGHT_KIND < 0:   # no fused kernel for this cost function / a user-defined CostWeight
+            if kind is None or not _fused_weight(kind, cf.weight.WEIGHT_KIND):   # no fused kernel for this cost function / its CostWeight
                 self.generic.append(f)
                 continue
-            key = (kind, cf.weight.WEIGHT_KIND, cf.dim(), int(getattr(cf, "robust_kind", 0)))
+            grid = tuple(cf.sdf_data.tensor.shape[1:]) if kind in _COLLISION_KINDS else None   # the kernels take one grid shape per group
+            key = (kind, cf.weight.WEIGHT_KIND, cf.dim(), int(getattr(cf, "robust_kind", 0)), grid)
             groups.setdefault(key, []).append(f)
         self.groups: List[_Group] = []
         dev = self.device
-        for (kind, wkind, dim, robust), idx in groups.items():
+        for (kind, wkind, dim, robust, grid), idx in groups.items():
             g = _Group(kind, wkind, dim, idx)
-            g.robust = robust
+            g.robust, g.grid = robust, grid
             ii = np.array(idx, dtype=np.int64)
-            bp = np.zeros((g.K, 2), dtype=np.int32)
+            bp = np.zeros((g.K, 4 if kind in _FOUR_VAR_KINDS else 2), dtype=np.int32)
             for r, f in enumerate(idx):
                 p = S.block_pointers[f]
                 bp[r, : len(p)] = p
@@ -243,10 +257,12 @@ class Engine:
 
         for g in self.groups:
             x0, x1, aux, w = [], [], [], []
+            x2, x3 = [], []
             extra = [[], [], []]
             n_extra = len(self._aux_of[g.cost_indices[0]]) - 1
             bs = np.zeros((g.K, 4), dtype=np.int32)
             bs2 = np.zeros((g.K, 3), dtype=np.int32)
+            bs3 = np.zeros((g.K, 2), dtype=np.int32)
             for r, f in enumerate(g.cost_indices):
                 cf = self.costs[f]
                 ov = cf.optim_vars
@@ -256,11 +272,20 @@ class Engine:
                 tw = aux_tensor(cf.weight.weight_tensor())
                 x0.append(t0); x1.append(t1); aux.append(auxs[0]); w.append(tw)
                 bs[r] = (bstride(t0), bstride(t1), bstride(auxs[0]), bstride(tw))
+                if g.kind in _FOUR_VAR_KINDS:
+                    t2, t3 = optim_tensor(ov[2]), optim_tensor(ov[3])
+                    x2.append(t2); x3.append(t3)
+                    bs3[r] = (bstride(t2), bstride(t3))
+                if g.grid is not None and tuple(auxs[1].shape[1:]) != g.grid:
+                    raise ValueError(f"{cf.name}: sdf_data changed shape from {g.grid} to {tuple(auxs[1].shape[1:])} after the objective was "
+                                     "compiled; add the cost function again (or use maps of one shape)")
                 for q in range(n_extra):
                     extra[q].append(auxs[1 + q])
                     bs2[r, q] = bstride(auxs[1 + q])
             keep = dict(x0=self._ptr_array(x0), x1=self._ptr_array(x1), aux=self._ptr_array(aux), w=self._ptr_array(w),
-                        bstride=_dev(bs, self.device), tensors=(x0, x1, aux, w, extra))
+                        bstride=_dev(bs, self.device), tensors=(x0, x1, aux, w, extra, x2, x3))
+            if x2:
+                keep["x2"], keep["x3"], keep["bstride3"] = self._ptr_array(x2), self._ptr_array(x3), _dev(bs3, self.device)
             ex = [self._ptr_array(extra[q]) if n_extra > q else None for q in range(3)]
             keep["extra"] = ex
             keep["bstride2"] = _dev(bs2, self.device)
@@ -278,7 +303,10 @@ class Engine:
                 aux2=ex[0].data_ptr() if ex[0] is not None else None, aux3=ex[1].data_ptr() if ex[1] is not None else None,
                 aux4=ex[2].data_ptr() if ex[2] is not None else None, bstride2=keep["bstride2"].data_ptr(),
                 robust_kind=g.robust, reserved0=0, log_radius=lr_ptr.data_ptr() if lr_ptr is not None else None,
-                bstride_lr=lr_bs.data_ptr() if lr_bs is not None else None)
+                bstride_lr=lr_bs.data_ptr() if lr_bs is not None else None,
+                x2=keep["x2"].data_ptr() if "x2" in keep else None, x3=keep["x3"].data_ptr() if "x3" in keep else None,
+                bstride3=keep["bstride3"].data_ptr() if "bstride3" in keep else None,
+                sdf_rows=g.grid[0] if g.grid is not None else 0, sdf_cols=g.grid[1] if g.grid is not None else 0)
             g.bound[which] = (st, keep)
         # NOTE: _bind may itself rebind non-contiguous tensors (bumping the counter); read it afterwards.
         self._bind_stamp[which] = Variable._global_updates
@@ -395,7 +423,8 @@ class Engine:
 
     def _user_costs(self, ids) -> bool:
         """True if any of these cost functions is a user-defined subclass (own error() / jacobians()): those run per cost function."""
-        return any(self.costs[f]._user_defined("jacobians") or self.costs[f]._user_defined("error") or self.costs[f].weight.WEIGHT_KIND < 0
+        return any(self.costs[f]._user_defined("jacobians") or self.costs[f]._user_defined("error")
+                   or self.costs[f].weight.WEIGHT_KIND not in (_WEIGHT_SCALE, _WEIGHT_DIAGONAL)
                    or getattr(getattr(self.costs[f], "cost_function", None), "_user_defined", lambda w: False)("jacobians") for f in ids)
 
     def _route(self, which: str):
